@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the HyperReel per-ray rendering hot path on B200 (contract: see the task prompt / DESIGN.md section 5).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (sample net -> intersect -> VM gather -> decode -> composite) over one
 synthetic batch of 65 536 rays x 32 samples per GPU, Technicolor-shape model (technicolor_z_plane: C_in=8,
@@ -179,7 +179,7 @@ def time_oracle(cfg, ds, sd, sig, hb, steps: int, warmup: int, rays_n: int, devi
     """The reference's op sequence restated (oracle port, same torch ops as the reference: F.grid_sample gathers, boolean-
     mask compaction, cumprod), eager PyTorch.  device='cpu': all usable host threads.  device='cuda': the same eager ops on
     the B200 -- the "beat eager PyTorch on the same GPU" baseline of SURVEY.md 2.3.  Returns (Mrays/s from the median step,
-    median ms, threads)."""
+    median ms, threads, rgb of the last step)."""
     import torch
     from oracle.hyperreel_oracle import HyperReelOracle
 
@@ -194,14 +194,14 @@ def time_oracle(cfg, ds, sd, sig, hb, steps: int, warmup: int, rays_n: int, devi
             if dev.type == "cuda":
                 torch.cuda.synchronize()
             t0 = time.perf_counter()
-            orc.render(rays.clone())
+            rgb = orc.render(rays.clone())
             if dev.type == "cuda":
                 torch.cuda.synchronize()
             if i >= warmup:
                 ts.append(time.perf_counter() - t0)
     ts.sort()
     med = ts[len(ts) // 2]
-    return rays_n / med / 1e6, med * 1e3, threads
+    return rays_n / med / 1e6, med * 1e3, threads, rgb
 
 
 def cpu_baseline_object(mrays, cores, sig, extra=""):
@@ -216,7 +216,9 @@ def run_reference(args):
         return
     hb, cfg, ds, sig, sd = build_workload()
     steps, warm = max(args.steps, 1), max(min(args.warmup, 2), 1)
-    mrays, ms, cores = time_oracle(cfg, ds, sd, sig, hb, steps, warm, CPU_SAMPLE_RAYS)
+    mrays, ms, cores, rgb = time_oracle(cfg, ds, sd, sig, hb, steps, warm, CPU_SAMPLE_RAYS)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"rgb": rgb})
     line = {
         "impl": "reference", "metric": METRIC, "value": mrays, "unit": "Mrays/s",
         "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True,
@@ -248,16 +250,27 @@ def make_render(hb, cfg, ds, sd, mlp=None):
 
 
 def timed_steps(torch, step, steps, flush):
+    """Total ms of `steps` timed calls of `step`, and what the last call returned."""
     evs = []
+    out = None
     for _ in range(steps):
         flush.zero_()  # evict L2 between timed iterations
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         a.record()
-        step()
+        out = step()
         b.record()
         evs.append((a, b))
     torch.cuda.synchronize()
-    return sum(a.elapsed_time(b) for a, b in evs)
+    return sum(a.elapsed_time(b) for a, b in evs), out
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each output array as `<out_dir>/<name>.npy` (float32), so that two builds can be compared output for output."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy())
 
 
 def kernel_times(torch, model, step, steps, flush):
@@ -301,7 +314,7 @@ def run_extra_workloads(torch, hb, dev, flush, steps, peak, peak_src):
         for _ in range(3):
             step()
         torch.cuda.synchronize()
-        ms = timed_steps(torch, step, steps, flush) / steps
+        ms = timed_steps(torch, step, steps, flush)[0] / steps
         tm = kernel_times(torch, model, step, steps, flush)
         out[key] = {"workload": spec["what"], "rays": n, "samples_per_ray": sig.n_samples, "value": n / (ms * 1e-3) / 1e6,
                     "unit": "Mrays/s", "ms_per_step": ms, "steps": steps,
@@ -414,7 +427,7 @@ def run_ours(args):
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize()
-        total_ms = timed_steps(torch, step, args.steps, flush)
+        total_ms, last_out = timed_steps(torch, step, args.steps, flush)
         if world > 1:
             dist.barrier()
         launches = model.launch_count() - launches0
@@ -426,6 +439,9 @@ def run_ours(args):
             break
         remeasured = True
         time.sleep(2.0)
+    if args.dump_outputs and rank == 0:  # copied now: later passes reuse the model's buffers
+        dump_outputs(args.dump_outputs, {"rgb": last_out})
+    del last_out
     # per-kernel durations for the roofline: a second pass with the library's CUDA events around each kernel (kept out of
     # the headline loop so the event records do not sit between the two kernels of a step)
     tm = kernel_times(torch, model, step, args.steps, flush)
@@ -473,7 +489,7 @@ def run_ours(args):
             assert torch.equal(got[lo:lo + 4096], render(rs[lo:lo + 4096])["rgb"]), "strong-scaling tiles differ from a local re-render"
             dist.barrier()
             k = max(3, args.steps // 4)
-            ms = torch.tensor([timed_steps(torch, sstep, k, flush) / k], device=dev, dtype=torch.float64)
+            ms = torch.tensor([timed_steps(torch, sstep, k, flush)[0] / k], device=dev, dtype=torch.float64)
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
             strong.append({"rays_total": total, "rays_per_gpu": total // world, "ms_per_step": float(ms.item()),
                            "value": total / (float(ms.item()) * 1e-3) / 1e6, "unit": "Mrays/s", "steps": k})
@@ -497,7 +513,7 @@ def run_ours(args):
         assert torch.equal(got[lo:lo + 4096], frender(fr[lo:lo + 4096])["rgb"]), "frame tiles differ from a local re-render"
         dist.barrier()
         k = 3
-        ms = torch.tensor([timed_steps(torch, fstep, k, flush) / k], device=dev, dtype=torch.float64)
+        ms = torch.tensor([timed_steps(torch, fstep, k, flush)[0] / k], device=dev, dtype=torch.float64)
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         frame = {"workload": "Neural-3D shape (BASELINE config 4): full 2704x2028 frame, 64 samples/ray, grid 823x617x514, K=12, comps [8,4,4], "
                              "SH-27, ray-sharded over the ranks through render_sharded", "rays_total": total,
@@ -525,7 +541,7 @@ def run_ours(args):
             extras["train_step"] = {"unavailable": repr(e)[:300]}
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         try:  # the reference's op sequence, eager PyTorch, on this same B200 (full 65 536-ray batch)
-            mr, ms, _ = time_oracle(cfg, ds, sd, sig, hb, 5, 2, n, device=f"cuda:{local}")
+            mr, ms, _, _ = time_oracle(cfg, ds, sd, sig, hb, 5, 2, n, device=f"cuda:{local}")
             baselines["torch_eager_b200"] = {"value": mr, "unit": "Mrays/s", "ms_per_step": ms, "rays": n,
                                              "what": "oracle port (the reference's torch op sequence: grid_sample gathers, mask compaction, cumprod) "
                                                      "run eagerly on cuda:0, fp32, median of 5 after 2 warm-ups; a stated baseline"}
@@ -537,7 +553,7 @@ def run_ours(args):
         peak, peak_src = measured_peaks()
         cpu = None
         if world == 1 and not args.no_cpu_baseline:
-            mr, _, cores = time_oracle(cfg, ds, sd, sig, hb, 5, 1, CPU_SAMPLE_RAYS)
+            mr, _, cores, _ = time_oracle(cfg, ds, sd, sig, hb, 5, 1, CPU_SAMPLE_RAYS)
             cpu = cpu_baseline_object(mr, cores, sig, extra=" of 5 after 1 warm-up")
         # sample net (tensor-core bound): algorithmic MACs of the six Linear layers x 3 split products x 2 flop
         macs = sum(o * i for o, i in sig.mlp_layer_shapes)
@@ -596,6 +612,8 @@ def main():
     ap.add_argument("--rays", type=int, default=RAYS_PER_GPU)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the rgb the timed path returned in its last timed step as DIR/rgb.npy (float32)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

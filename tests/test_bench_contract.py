@@ -44,3 +44,20 @@ def test_reference_arm_prints_the_contract_line():
     assert line["cpu_baseline"]["kind"] == "port" and line["cpu_baseline"]["cores"] >= 1
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["e2e"]["d2h_bytes_per_step"] == 0
     assert line["value"] > 0 and line["config"]["workload"].startswith("technicolor_z_plane")
+
+
+def test_dump_outputs_writes_the_same_rgb_on_every_run(tmp_path):
+    """`--dump-outputs DIR` writes the rgb of the last timed step as DIR/rgb.npy; the inputs are seeded, so two runs with the
+    same arguments write the same array (what makes two builds comparable output for output)."""
+    import numpy as np
+
+    env = dict(os.environ, HR_BENCH_CPU_RAYS="256")
+    got = []
+    for i in range(2):
+        d = tmp_path / f"run{i}"
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "1",
+                              "--dump-outputs", str(d)], capture_output=True, text=True, env=env, timeout=600)
+        assert out.returncode == 0, out.stderr[-2000:]
+        got.append(np.load(d / "rgb.npy"))
+    assert got[0].shape == (256, 3) and got[0].dtype == np.float32 and np.isfinite(got[0]).all()
+    assert np.array_equal(got[0], got[1])

@@ -1,5 +1,6 @@
 """Host-side logic that needs no GPU: config lowering, registry surface, chunk loop, state_dict layout,
 C-ABI symbol table."""
+import copy
 import os
 import re
 
@@ -10,6 +11,7 @@ import hyperreel_b200 as hb
 from hyperreel_b200 import lib as L
 from hyperreel_b200.signature import UnsupportedPipeline, lower
 from hyperreel_b200.state import n_to_reso, seeded_state_dict
+from tests import reference_pins
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -159,18 +161,21 @@ def test_lowering_of_the_f3_families():
     assert c.isect_type == L.ISECT_SPHERE and c.dynamic == 1 and c.contract_type == L.CONTRACT_MIPNERF
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/conf/experiment/model"), reason="reference checkout not present")
+def _shipped_yaml(name):
+    """One of the reference's shipped model YAMLs (conf/experiment/model/<name>.yaml), from the stored record."""
+    return hb.to_cfg(copy.deepcopy(reference_pins.model_yamls()[name]))
+
+
 def test_shipped_model_yamls_that_lower_to_the_fused_path():
     """Coverage ledger over the reference's 51 shipped model YAMLs: these must lower (DESIGN.md section 7 lists why the
     rest are rejected)."""
-    import glob
     ds = {"num_keyframes": 12, "num_frames": 50, "near": 0.5, "far": 10.0, "depth_range": [0.5, 10.0], "name": "x", "collection": "y",
           "bbox_min": [-1.5, -1.25, -1.0], "bbox_max": [1.5, 1.25, 1.0], "total_images_per_frame": 5, "val_all": True}
     ok = set()
-    for f in sorted(glob.glob("/root/reference/conf/experiment/model/*.yaml")):
+    for name in sorted(reference_pins.model_yamls()):
         try:
-            lower(hb.load_model_yaml(f), ds)
-            ok.add(os.path.basename(f)[:-5])
+            lower(_shipped_yaml(name), ds)
+            ok.add(name)
         except (UnsupportedPipeline, TypeError):  # bom_z_plane.yaml is an empty file
             pass
     expected = {
@@ -248,33 +253,30 @@ def test_system_loads_shrunk_grid_checkpoint_shapes():
 def test_lowering_of_the_round_2_families():
     """Voxel grids (per-axis sample tables, interleaved), plane grids, 256 samples per ray, the per-camera colour transform and
     cascaded (point_prediction) pipelines, lowered from the reference's own YAML files."""
-    ref = "/root/reference/conf/experiment/model"
-    if not os.path.isdir(ref):
-        pytest.skip("reference checkout not present")
-    ds = {"num_keyframes": 12, "num_frames": 50, "near": 0.5, "far": 10.0, "depth_range": [0.5, 10.0], "name": "x", "collection": "y",
+    ds ={"num_keyframes": 12, "num_frames": 50, "near": 0.5, "far": 10.0, "depth_range": [0.5, 10.0], "name": "x", "collection": "y",
           "bbox_min": [-1.5, -1.25, -1.0], "bbox_max": [1.5, 1.25, 1.0], "total_images_per_frame": 5, "val_all": True}
-    c = lower(hb.load_model_yaml(f"{ref}/donerf_voxel.yaml"), ds).cfg
+    c = lower(_shipped_yaml("donerf_voxel"), ds).cfg
     assert c.isect_type == L.ISECT_VOXEL and c.n_samples == 48 and c.isect_axes == 3 and c.n_z == 1
     # sample s = plane s // 3 of axis s % 3: first / last plane of every axis are the (contracted) dataset bounds
     assert c.samples[0] < 0 < c.samples[45] and c.samples[1] < 0 < c.samples[46] and c.samples[2] < 0 < c.samples[47]
     assert all(abs(c.z_scale3[a] - abs(c.samples[3 + a] - c.samples[a])) < 1e-6 for a in range(3))
-    c = lower(hb.load_model_yaml(f"{ref}/shiny_z_deformable.yaml"), ds).cfg
+    c = lower(_shipped_yaml("shiny_z_deformable"), ds).cfg
     assert c.isect_type == L.ISECT_PLANE and c.n_z == 4 and c.isect_axes == 1 and list(c.plane_normal)[:3] == [0.0, 0.0, 1.0]
     assert c.plane_normal_scale == 1.0
-    sig = lower(hb.load_model_yaml(f"{ref}/neural_3d_z_plane_static.yaml"), ds)
+    sig = lower(_shipped_yaml("neural_3d_z_plane_static"), ds)
     assert sig.n_samples == 256 and sig.cfg.mlp_out == 256 * 14 and sig.cfg.dynamic == 0
-    sig = lower(hb.load_model_yaml(f"{ref}/immersive_z_plane.yaml"), ds)
+    sig = lower(_shipped_yaml("immersive_z_plane"), ds)
     assert sig.cfg.n_color_views == 5 and sig.cfg.c_in == 8 and sig.color_views == 5 and sig.color_embedding_index > 0
     assert abs(sig.cfg.act_ctransform.inner_fac - 0.1) < 1e-7
     off = dict(ds, val_all=False)
-    assert lower(hb.load_model_yaml(f"{ref}/immersive_z_plane.yaml"), off).cfg.n_color_views == 0  # ColorTransformEmbedding is a no-op then
-    sig = lower(hb.load_model_yaml(f"{ref}/technicolor_cascaded.yaml"), ds)
+    assert lower(_shipped_yaml("immersive_z_plane"), off).cfg.n_color_views == 0  # ColorTransformEmbedding is a no-op then
+    sig = lower(_shipped_yaml("technicolor_cascaded"), ds)
     c = sig.cfg
     assert c.cascade == 1 and c.pre_samples == 8 and c.n_samples == 32 and sig.net_index == 2
     assert sig.pre_layer_shapes[-1] == (8, 256) and sig.mlp_layer_shapes[-1] == (c.mlp_out // 8, 256)
     assert list(c.pt_src) == [0, 1, 2, 3, 4, 5, 9, -1]  # points, viewdirs, times
     assert c.pre_mlp_mode == c.mlp_mode and c.pre_near == float("-inf")  # mask.stop_iters: -1 -> nothing masked
-    c = lower(hb.load_model_yaml(f"{ref}/shiny_z_plane_cascaded.yaml"), ds).cfg
+    c = lower(_shipped_yaml("shiny_z_plane_cascaded"), ds).cfg
     assert c.cascade == 1 and c.pre_mlp_mode == L.MLP_ZERO  # zero ray net: the first stage is the bare z-planes
     sd = seeded_state_dict(sig, seed=1)
     assert sd["model.embedding_model.embeddings.2.net.layers.0.0.weight"].shape == (256, 24)

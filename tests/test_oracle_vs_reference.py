@@ -1,13 +1,14 @@
-"""Live pin: the oracle and the built-in configs against the reference checkout itself (skipped where
-/root/reference is absent, e.g. on the GPU box -- the committed golden vectors cover that case)."""
+"""The oracle, the built-in configs and the host code against what the unmodified reference computes, recorded from the
+reference itself by tests/golden/make_golden_reference_pins.py (tests/golden/reference_pins.npz): every check here
+holds this project to the reference without needing a reference checkout."""
+import copy
+
 import pytest
 import torch
 
-from oracle import ref_shim
 from oracle.hyperreel_oracle import HyperReelOracle
+from tests import reference_pins as P
 from tests.cases import build_case
-
-pytestmark = pytest.mark.skipif(not ref_shim.reference_available(), reason="reference checkout not present")
 
 
 def _floatify(o):
@@ -31,11 +32,23 @@ def _key_order(o):
     return None
 
 
+def _yaml(name):
+    """A shipped model YAML of the reference, as the product reads it (hyperreel_b200.load_model_yaml)."""
+    import hyperreel_b200 as hb
+
+    return hb.to_cfg(copy.deepcopy(P.model_yamls()[name]))
+
+
+def _close(want, got, tol, what=None):
+    assert tuple(want.shape) == tuple(got.shape), (what, tuple(want.shape), tuple(got.shape))
+    assert float((want - got).abs().max()) <= tol, what
+
+
 @pytest.mark.parametrize("name", ["technicolor_z_plane", "neural_3d_z_plane", "donerf_sphere", "shiny_z_plane_tiny"])
 def test_builtin_config_equals_reference_yaml(name):
     from hyperreel_b200 import configs
     from hyperreel_b200.config import to_plain
-    ref = _floatify(ref_shim.load_reference_yaml(name))
+    ref = _floatify(P.model_yamls()[name])
     mine = _floatify(to_plain(configs.BUILTIN[name]()))
     assert ref == mine
     # ordered sections: embedding order, head order and param-group order are semantic
@@ -45,82 +58,60 @@ def test_builtin_config_equals_reference_yaml(name):
     assert list(e_ref["ray_prediction_0"]["params"]) == list(e_mine["ray_prediction_0"]["params"])
 
 
-@pytest.mark.parametrize("name", ["technicolor_trained", "neural3d_trained", "donerf_s16"])
+@pytest.mark.parametrize("name", P.FRESH_CASES)
 def test_oracle_matches_live_reference_on_fresh_rays(name):
-    case = build_case(name, n=777)
-    ref = ref_shim.build_reference(case.model_cfg_plain, case.dataset)
-    missing, unexpected = ref.load_state_dict(case.state_dict, strict=False)
-    assert not unexpected
-    out = ref_shim.run_reference(ref, case.rays.clone(), chunk=200, capture=True)
+    case = build_case(name, n=P.FRESH_RAYS)
     st = {}
     rgb = HyperReelOracle(case.model_cfg_plain, case.dataset, case.state_dict).render(case.rays.clone(), st)
-    assert (rgb - out["rgb"]).abs().max() <= 2e-6
-    n, S = case.rays.shape[0], case.n_samples
-    assert (st["points"].reshape(n, -1) - out["_embed"]["points"]).abs().max() <= 2e-6
-    assert (st["distances"] - out["_embed"]["distances"]).abs().max() <= 2e-6
+    n = case.rays.shape[0]
+    _close(P.array(f"fresh/{name}/rgb"), rgb, 2e-6)
+    _close(*P.sampled(f"fresh/{name}/points", st["points"].reshape(n, -1)), 2e-6)
+    _close(*P.sampled(f"fresh/{name}/distances", st["distances"].reshape(n, -1)), 2e-6)
 
 
-@pytest.mark.parametrize("name", ["technicolor_trained", "neural3d_trained", "donerf_trained", "immersive_sphere_new",
-                                  "donerf_cylinder", "technicolor_bbox"])
+@pytest.mark.parametrize("name", P.EDGE_CASES)
 def test_oracle_matches_reference_on_crafted_edge_rays(name):
     """The rays of tests/test_edge_rays_gpu.py (plane-parallel, keyframe boundaries, far / centred origins, un-normalised
     directions): the oracle must still equal the unmodified reference there before it may judge the CUDA path."""
-    ref_shim.install()
-    from nlf.rendering import render_chunked
     from tests.test_edge_rays_gpu import craft
 
     case = build_case(name)
     rays = craft(case)
-    ref = ref_shim.build_reference(case.model_cfg_plain, case.dataset)
-    ref.load_state_dict(case.state_dict, strict=False)
-    with torch.no_grad():
-        a = render_chunked(rays.clone(), ref, {}, rays.shape[0])["rgb"]
+    a = P.array(f"edge/{name}/rgb")
     b = HyperReelOracle(case.model_cfg_plain, case.dataset, case.state_dict).render(rays.clone())
     assert torch.isfinite(a).all()
     assert float((a.reshape(b.shape) - b).abs().max()) <= 2e-6
 
 
 def test_oracle_matches_reference_on_every_shipped_yaml_that_lowers():
-    """Every model YAML the reference ships that the fused path accepts (34 of 51): build the unmodified reference from the
-    YAML itself (grid shrunk to 24^3 for speed), load seeded parameters, and hold the oracle to it on seeded rays.  This
+    """Every model YAML the reference ships that the fused path accepts (45 of 52): the unmodified reference built from the
+    YAML itself (grid shrunk to 24^3 for speed) rendered seeded rays with seeded parameters; the oracle must equal it.  This
     pins the oracle's reading of the real configuration files, not only of the built-ins and their variants."""
-    import glob
-    import os
-
     import hyperreel_b200 as hb
     from hyperreel_b200.config import to_plain
     from hyperreel_b200.signature import UnsupportedPipeline
     from hyperreel_b200.state import seeded_state_dict
 
-    ref_shim.install()
-    from nlf.rendering import render_chunked
-
-    ds = {"num_keyframes": 12, "num_frames": 50, "near": 0.5, "far": 10.0, "depth_range": [0.5, 10.0], "name": "x", "collection": "y",
-          "bbox_min": [-1.5, -1.25, -1.0], "bbox_max": [1.5, 1.25, 1.0], "total_images_per_frame": 5, "val_all": True}
-    checked, nonzero = 0, 0
-    for f in sorted(glob.glob(os.path.join(ref_shim.REFERENCE_ROOT, "conf/experiment/model/*.yaml"))):
-        cfg = hb.load_model_yaml(f)
+    checked, nonzero = [], 0
+    for name in sorted(P.model_yamls()):
+        cfg = _yaml(name)
         if cfg is None:  # bom_z_plane.yaml is empty
             continue
-        cfg.color.net.N_voxel_init = 24 ** 3
-        cfg.color.net.N_voxel_final = 24 ** 3
+        cfg.color.net.N_voxel_init = P.SHIPPED_GRID
+        cfg.color.net.N_voxel_final = P.SHIPPED_GRID
         try:
-            sig = hb.lower(cfg, ds)
+            sig = hb.lower(cfg, P.DS_R2)
         except UnsupportedPipeline:
             continue
         sd = seeded_state_dict(sig, seed=3, density_gain=30.0)
         rays = hb.rays.for_signature(sig, 48, seed=9)
-        plain = to_plain(cfg)
-        ref = ref_shim.build_reference(plain, ds)
-        _, unexpected = ref.load_state_dict(sd, strict=False)
-        assert not unexpected, (f, unexpected)
-        with torch.no_grad():
-            a = render_chunked(rays.clone(), ref, {}, rays.shape[0])["rgb"]
-        b = HyperReelOracle(plain, ds, sd).render(rays.clone())
-        assert float((a.reshape(b.shape) - b).abs().max()) <= 2e-6, os.path.basename(f)
-        checked += 1
+        a = P.array(f"shipped/{name}/rgb")
+        b = HyperReelOracle(to_plain(cfg), P.DS_R2, sd).render(rays.clone())
+        assert float((a.reshape(b.shape) - b).abs().max()) <= 2e-6, name
+        checked.append(name)
         nonzero += int(float(b.abs().max()) > 0)
-    assert checked >= 45 and nonzero >= 40
+    assert [k.split("/")[1] for k in P.keys("shipped/")] == checked  # every YAML the reference rendered is checked
+    assert len(checked) >= 45 and nonzero >= 40
 
 
 def test_six_shipped_yamls_do_not_run_in_the_reference_itself():
@@ -128,72 +119,51 @@ def test_six_shipped_yamls_do_not_run_in_the_reference_itself():
     shiny_z_tensorf (`z` is not a registered intersect type), donerf_z / shiny_z_depth (`epipolar` is not a registered embedding
     type) and blender_voxel (its ray_prediction has no `params`) fail inside the unmodified reference, so no implementation can
     be held to them; together with the empty bom_z_plane.yaml they are excluded from the denominator in DESIGN.md section 7.
-    (The YAMLs are read like Hydra / OmegaConf reads them: `1e-4` is a float, hyperreel_b200/config.py:_yaml_loader.)"""
+    The record holds the error the reference raised for each; the fused path rejects each of them up front."""
     import hyperreel_b200 as hb
-    from hyperreel_b200.config import to_plain
+    from hyperreel_b200.signature import UnsupportedPipeline
 
-    ref_shim.install()
-    from nlf.rendering import render_chunked
-
-    ds = {"num_keyframes": 12, "num_frames": 50, "near": 0.5, "far": 10.0, "depth_range": [0.5, 10.0], "name": "x", "collection": "y"}
-    for name in ("catacaustics_sphere", "refnerf_sphere", "shiny_z_tensorf", "donerf_z", "shiny_z_depth", "blender_voxel"):
-        cfg = hb.load_model_yaml(f"{ref_shim.REFERENCE_ROOT}/conf/experiment/model/{name}.yaml")
+    fails = P.meta("reference_fails")
+    assert sorted(fails) == sorted(P.REFERENCE_FAILS)
+    for name in P.REFERENCE_FAILS:
+        assert fails[name] is not None and fails[name][0] in ("RuntimeError", "KeyError", "AttributeError", "TypeError"), name
+        cfg = _yaml(name)
         cfg.color.net.N_voxel_init = cfg.color.net.N_voxel_final = 16 ** 3
-        rays = torch.randn(8, 6) * 0.3
-        rays[:, 3:6] = torch.nn.functional.normalize(torch.randn(8, 3), dim=-1)
-        with pytest.raises((RuntimeError, KeyError, AttributeError, TypeError)):
-            ref = ref_shim.build_reference(to_plain(cfg), ds)
-            with torch.no_grad():
-                render_chunked(rays, ref, {}, 8)
+        with pytest.raises(UnsupportedPipeline):
+            hb.lower(cfg, P.DS)
 
 
-@pytest.mark.parametrize("name", ["technicolor_z_plane", "donerf_sphere"])
+@pytest.mark.parametrize("name", P.UPSAMPLE_YAMLS)
 def test_grid_upsampling_and_regulariser_terms_match_the_reference(name):
     """The training-schedule pieces mirrored on the host (SURVEY.md 8 row f1): `upsample_volume_grid` re-samples every table
     exactly like the reference's (tensorf_base.py:1151-1188, tensorf_dynamic.py:394-441), and the TensoRF regulariser's terms
     (density_L1, TV on the space planes; nlf/regularizers/tensorf.py:14-96) agree on the same parameters."""
     import hyperreel_b200 as hb
-    from hyperreel_b200.config import to_plain
     from hyperreel_b200.state import _Color, seeded_state_dict
     from hyperreel_b200.system import TVLoss
 
-    ref_shim.install()
-    # nlf/regularizers/__init__.py imports every regulariser (and through them the datasets): import tensorf.py alone, with
-    # a stand-in for the base class it derives from
-    import sys
-    import types
-    if "nlf.regularizers" not in sys.modules:
-        pkg = types.ModuleType("nlf.regularizers")
-        pkg.__path__ = [f"{ref_shim.REFERENCE_ROOT}/nlf/regularizers"]
-        sys.modules["nlf.regularizers"] = pkg
-        base = types.ModuleType("nlf.regularizers.base")
-        base.BaseRegularizer = type("BaseRegularizer", (torch.nn.Module,), {})
-        sys.modules["nlf.regularizers.base"] = base
-    from nlf.regularizers.tensorf import TVLoss as RefTV
-
-    ds = {"num_keyframes": 12, "num_frames": 50, "near": 0.5, "far": 10.0, "depth_range": [0.5, 10.0], "name": "x", "collection": "y"}
-    cfg = hb.load_model_yaml(f"{ref_shim.REFERENCE_ROOT}/conf/experiment/model/{name}.yaml")
+    cfg = _yaml(name)
     cfg.color.net.N_voxel_init, cfg.color.net.N_voxel_final = 12 ** 3, 20 ** 3
-    sig = hb.lower(cfg, ds)
+    sig = hb.lower(cfg, P.DS)
     sd = seeded_state_dict(sig, seed=4)
-    ref = ref_shim.build_reference(to_plain(cfg), ds)
-    ref.load_state_dict(sd, strict=False)
-    rnet = ref.model.color_model.net
+    k = f"upsample/{name}/"
     mine = _Color(sig, hb.state.default_grid(sig))
     mine.load_state_dict({k[len("model.color_model."):]: v for k, v in sd.items() if k.startswith("model.color_model.")}, strict=False)
-    assert abs(float(rnet.density_L1()) - float(mine.net.density_L1())) <= 1e-7
-    assert abs(float(rnet.TV_loss_density(RefTV())) - float(mine.net.TV_loss_density(TVLoss()))) <= 1e-9
-    assert abs(float(rnet.TV_loss_app(RefTV())) - float(mine.net.TV_loss_app(TVLoss()))) <= 1e-7
+    l1, tv_density, tv_app = P.array(k + "terms").tolist()
+    assert abs(l1 - float(mine.net.density_L1())) <= 1e-7
+    assert abs(tv_density - float(mine.net.TV_loss_density(TVLoss()))) <= 1e-9
+    assert abs(tv_app - float(mine.net.TV_loss_app(TVLoss()))) <= 1e-7
     # the schedule: same voxel counts, same re-sampled tables
-    assert [int(v) for v in rnet.N_voxel_list] == [int(v) for v in mine.net.N_voxel_list]
+    assert P.array(k + "n_voxel_list").tolist() == [int(v) for v in mine.net.N_voxel_list]
     reso = hb.state.n_to_reso(int(mine.net.N_voxel_list[0]), torch.tensor(cfg.color.net.aabb))
-    rnet.upsample_volume_grid(reso)
     mine.net.upsample_volume_grid(reso)
-    assert rnet.gridSize.tolist() == mine.net.gridSize.tolist() == list(reso)
+    assert P.array(k + "grid").tolist() == mine.net.gridSize.tolist() == list(reso)
     got = mine.state_dict()
-    for k, v in rnet.state_dict().items():
-        if any(t in k for t in ("plane", "line")):
-            assert torch.equal(v, got["net." + k]), k
+    tables = [t[len(k + "table/"):] for t in P.keys(k + "table/") if not t.endswith("#shape")]
+    assert tables
+    for t in tables:
+        want, have = P.sampled(k + "table/" + t, got["net." + t])
+        assert torch.equal(want, have), t
 
 
 def test_tensorf_regulariser_loss_sequence_matches_the_reference():
@@ -201,58 +171,24 @@ def test_tensorf_regulariser_loss_sequence_matches_the_reference():
     replaced by a stand-in): same loss over several calls -- including the reference's running-weight bookkeeping (the TV
     weights decay per call, the density TV term is counted again inside the appearance term) and the L1 switch at the first
     alpha-mask iteration."""
-    import sys
-    import types
-    from types import SimpleNamespace
-
     import hyperreel_b200 as hb
-    from hyperreel_b200.config import to_plain
     from hyperreel_b200.state import _Color, seeded_state_dict
     from hyperreel_b200.system import TensoRFRegularizer
 
-    ref_shim.install()
-    if "nlf.regularizers" not in sys.modules:
-        pkg = types.ModuleType("nlf.regularizers")
-        pkg.__path__ = [f"{ref_shim.REFERENCE_ROOT}/nlf/regularizers"]
-        sys.modules["nlf.regularizers"] = pkg
-        base = types.ModuleType("nlf.regularizers.base")
-        base.BaseRegularizer = type("BaseRegularizer", (torch.nn.Module,), {})
-        sys.modules["nlf.regularizers.base"] = base
-    from nlf.regularizers.tensorf import TensoRF as RefReg
-
-    class Base(torch.nn.Module):  # what BaseRegularizer provides to this class: the system handle and the iteration counter
-        def __init__(self, system, cfg):
-            super().__init__()
-            self._system, self.cur_iter = [system], 0
-
-        def get_system(self):
-            return self._system[0]
-
-        def set_iter(self, i):
-            self.cur_iter = i
-
-    RefReg.__bases__ = (Base,)
-    ds = {"num_keyframes": 12, "num_frames": 50, "near": 0.5, "far": 10.0, "depth_range": [0.5, 10.0], "name": "x", "collection": "y"}
-    cfg = hb.load_model_yaml(f"{ref_shim.REFERENCE_ROOT}/conf/experiment/model/technicolor_z_plane.yaml")
+    cfg = _yaml("technicolor_z_plane")
     cfg.color.net.N_voxel_init = cfg.color.net.N_voxel_final = 14 ** 3
-    sig = hb.lower(cfg, ds)
+    sig = hb.lower(cfg, P.DS)
     sd = seeded_state_dict(sig, seed=6)
-    ref = ref_shim.build_reference(to_plain(cfg), ds)
-    ref.load_state_dict(sd, strict=False)
-    system = SimpleNamespace(is_subdivided=False, render_fn=ref)
-    rcfg = ref_shim.to_attr({"type": "tensorf", "update_AlphaMask_list": [2], "lr_decay_target_ratio": 0.1, "n_iters": 50,
-                             "L1_weight_initial": 8e-5, "L1_weight_rest": 4e-5, "TV_weight_density": 0.05, "TV_weight_app": 0.05})
-    theirs = RefReg(system, rcfg)
-    mine = TensoRFRegularizer(dict(rcfg))
+    mine = TensoRFRegularizer(dict(P.REGULARISER_CFG))
     net = _Color(sig, hb.state.default_grid(sig))
     net.load_state_dict({k[len("model.color_model."):]: v for k, v in sd.items() if k.startswith("model.color_model.")}, strict=False)
-    for it in range(6):
-        theirs.set_iter(it)
+    theirs = P.array("regulariser/loss").tolist()
+    assert len(theirs) == P.REGULARISER_CALLS
+    for it, a in enumerate(theirs):
         mine.set_iter(it)
-        a = float(theirs._loss(None, None, 0))
         b = float(mine.loss(net.net))
         assert abs(a - b) <= 1e-7 * max(1.0, abs(a)), (it, a, b)
-    assert mine.L1_reg_weight == 4e-5 and abs(mine.TV_weight_density - theirs.TV_weight_density) < 1e-12
+    assert mine.L1_reg_weight == 4e-5 and abs(mine.TV_weight_density - float(P.array("regulariser/tv_weight_density"))) < 1e-12
 
 
 def test_oracle_stages_match_the_reference_on_the_round_2_families():
@@ -263,200 +199,142 @@ def test_oracle_stages_match_the_reference_on_the_round_2_families():
     from hyperreel_b200.config import to_plain
     from hyperreel_b200.state import seeded_state_dict
 
-    ds = {"num_keyframes": 12, "num_frames": 50, "near": 0.5, "far": 10.0, "depth_range": [0.5, 10.0], "name": "x", "collection": "y",
-          "bbox_min": [-1.5, -1.25, -1.0], "bbox_max": [1.5, 1.25, 1.0], "total_images_per_frame": 5, "val_all": True}
-    for name in ("catacaustics_voxel", "donerf_voxel", "shiny_z_deformable", "immersive_z_plane", "neural_3d_z_plane_static",
-                 "technicolor_z_plane_no_sample", "shiny_z_plane_cascaded", "shiny_z_plane_feedback", "shiny_z_tensorf_cascaded",
-                 "technicolor_cascaded"):
-        cfg = hb.load_model_yaml(f"{ref_shim.REFERENCE_ROOT}/conf/experiment/model/{name}.yaml")
+    for name in P.STAGE_YAMLS:
+        cfg = _yaml(name)
         cfg.color.net.N_voxel_init = cfg.color.net.N_voxel_final = 16 ** 3
-        sig = hb.lower(cfg, ds)
+        sig = hb.lower(cfg, P.DS_R2)
         sd = seeded_state_dict(sig, seed=5, density_gain=30.0)
         rays = hb.rays.for_signature(sig, 40, seed=3)
-        plain = to_plain(cfg)
-        ref = ref_shim.build_reference(plain, ds)
-        ref.load_state_dict(sd, strict=False)
-        out = ref_shim.run_reference(ref, rays.clone(), capture=True)
         st = {}
-        rgb = HyperReelOracle(plain, ds, sd).render(rays.clone(), st)
+        rgb = HyperReelOracle(to_plain(cfg), P.DS_R2, sd).render(rays.clone(), st)
         n = rays.shape[0]
-        assert float((rgb - out["rgb"].reshape(rgb.shape)).abs().max()) <= 2e-6, name
-        assert float((st["points"].reshape(n, -1) - out["_embed"]["points"].reshape(n, -1)).abs().max()) <= 2e-6, name
-        assert float((st["distances"].reshape(n, -1) - out["_embed"]["distances"].reshape(n, -1)).abs().max()) <= 2e-6, name
+        _close(P.array(f"stages/{name}/rgb"), rgb.reshape(n, 3), 2e-6, name)
+        _close(*P.sampled(f"stages/{name}/points", st["points"].reshape(n, -1)), 2e-6, name)
+        _close(*P.sampled(f"stages/{name}/distances", st["distances"].reshape(n, -1)), 2e-6, name)
 
 
-@pytest.mark.parametrize("name,gain", [("technicolor_z_plane", 40000.0), ("donerf_sphere", 40000.0)])
+@pytest.mark.parametrize("name,gain", P.ALPHA_CASES)
 def test_alpha_mask_update_and_shrink_match_the_reference(name, gain):
     """The pruning step of the training schedule (tensorf_base.py:379-429,1190-1232 / tensorf_dynamic.py:443-541): dense
     occupancy, mask, bounding box, cropped tables and corrected aabb equal the unmodified reference's on the same parameters;
     a second mask update (which, in the static net, consults the first mask) as well."""
     import hyperreel_b200 as hb
-    from hyperreel_b200.config import to_plain
     from hyperreel_b200.state import _Color, seeded_state_dict
 
-    ds = {"num_keyframes": 4, "num_frames": 6, "near": 0.5, "far": 10.0, "depth_range": [0.5, 10.0], "name": "x", "collection": "y"}
-    cfg = hb.load_model_yaml(f"{ref_shim.REFERENCE_ROOT}/conf/experiment/model/{name}.yaml")
+    cfg = _yaml(name)
     cfg.color.net.N_voxel_init = cfg.color.net.N_voxel_final = 13 ** 3
-    sig = hb.lower(cfg, ds)
-    sd = seeded_state_dict(sig, seed=8)
-    # occupancy confined to a corner region, so that the box of occupied voxels is a strict subset of the grid
-    # (empty for x in the lower half of the box: groups 0 and 1 have x as their planes' column axis, group 2 as its line's axis)
-    for k in list(sd):
-        if "density_plane" in k and "time" not in k and sd[k].numel() > 0:
-            t = sd[k].clone() * gain
-            if not k.endswith(".2"):
-                t[..., : t.shape[-1] // 2] = 0
-            sd[k] = t
-        if "density_line.2" in k and sd[k].numel() > 0:
-            t = sd[k].clone()
-            t[..., : t.shape[-2] // 2, :] = 0
-            sd[k] = t
-    ref = ref_shim.build_reference(to_plain(cfg), ds)
-    ref.load_state_dict(sd, strict=False)
-    rnet = ref.model.color_model.net
+    sig = hb.lower(cfg, P.DS_ALPHA)
+    sd = P.corner_occupancy(seeded_state_dict(sig, seed=8), gain)
     mine = _Color(sig, hb.state.default_grid(sig))
     mine.load_state_dict({k[len("model.color_model."):]: v for k, v in sd.items() if k.startswith("model.color_model.")}, strict=False)
-    reso = tuple(rnet.gridSize.tolist())
+    k = f"alpha/{name}/"
+    reso = tuple(P.array(k + "grid0").tolist())
+    assert reso == tuple(mine.net.gridSize.tolist())
+    a_ref = P.array(k + "dense_alpha")
     with torch.no_grad():
-        a_ref, _ = rnet.getDenseAlpha(reso)
         a_mine, _ = mine.net.getDenseAlpha(reso)
     # (the reference evaluates slab by slab, here in one batch: the same values up to the last bit or two)
-    assert float((a_ref - a_mine).abs().max()) <= 1e-6 and float(a_ref.max()) > 0.05 > 0.001 > float(a_ref.min())
-    box_ref = rnet.updateAlphaMask(reso)
+    _close(a_ref, a_mine, 1e-6)
+    assert float(a_ref.max()) > 0.05 > 0.001 > float(a_ref.min())
+    box_ref = P.array(k + "box")
     box_mine = mine.net.updateAlphaMask(reso)
     assert torch.equal(box_ref, box_mine)
-    assert torch.equal(rnet.alphaMask.alpha_volume, mine.net.alphaMask.volume)
-    rnet.shrink(box_ref)
+    assert torch.equal(P.array(k + "alpha_volume"), mine.net.alphaMask.volume)
     mine.net.shrink(box_mine)
-    assert rnet.gridSize.tolist() == mine.net.gridSize.tolist() and any(g < r for g, r in zip(rnet.gridSize.tolist(), reso))
-    assert torch.equal(rnet.aabb, mine.net.aabb)
+    grid = P.array(k + "grid").tolist()
+    assert grid == mine.net.gridSize.tolist() and any(g < r for g, r in zip(grid, reso))
+    assert torch.equal(P.array(k + "aabb"), mine.net.aabb)
     got = mine.state_dict()
-    for k, v in rnet.state_dict().items():
-        if any(t in k for t in ("plane", "line")):
-            assert torch.equal(v, got["net." + k]), k
-    reso2 = tuple(rnet.gridSize.tolist())
-    assert torch.equal(rnet.updateAlphaMask(reso2), mine.net.updateAlphaMask(reso2))
+    tables = [t[len(k + "table/"):] for t in P.keys(k + "table/") if not t.endswith("#shape")]
+    assert tables
+    for t in tables:
+        want, have = P.sampled(k + "table/" + t, got["net." + t])
+        assert torch.equal(want, have), t
+    reso2 = tuple(mine.net.gridSize.tolist())
+    assert torch.equal(P.array(k + "box2"), mine.net.updateAlphaMask(reso2))
 
 
 def test_lowered_constants_equal_the_reference_constructors_on_every_shipped_yaml():
     """hyperreel_b200.signature.lower (product host code) against the objects the unmodified reference builds from the same YAML
     and dataset facts: base primitives (`samples`), their spacing (`z_scale`), the mask bounds, the contraction radii, and the
     colour net's scalars -- for all 45 shipped model YAMLs that run, under two sets of dataset facts."""
-    import glob
-    import os
-
     import hyperreel_b200 as hb
     from hyperreel_b200 import lib as L
-    from hyperreel_b200.config import to_plain
     from hyperreel_b200.signature import UnsupportedPipeline
 
-    ref_shim.install()
-    facts = [
-        {"num_keyframes": 12, "num_frames": 50, "near": 0.5, "far": 10.0, "depth_range": [0.5, 10.0], "name": "x", "collection": "y",
-         "bbox_min": [-1.5, -1.25, -1.0], "bbox_max": [1.5, 1.25, 1.0], "total_images_per_frame": 5, "val_all": True},
-        {"num_keyframes": 7, "num_frames": 30, "near": 0.25, "far": 6.0, "depth_range": [0.75, 4.0], "name": "x", "collection": "y",
-         "bbox_min": [-0.5, -2.0, -1.5], "bbox_max": [2.5, 1.0, 0.5], "total_images_per_frame": 3, "val_all": False},
-    ]
+    records = {(r["name"], r["facts"]): r for r in P.meta("constants")}
     checked = 0
-    for f in sorted(glob.glob(os.path.join(ref_shim.REFERENCE_ROOT, "conf/experiment/model/*.yaml"))):
-        cfg = hb.load_model_yaml(f)
+    for name in sorted(P.model_yamls()):
+        cfg = _yaml(name)
         if cfg is None:
             continue
         cfg.color.net.N_voxel_init = cfg.color.net.N_voxel_final = 12 ** 3
-        for ds in facts:
+        for fi, ds in enumerate(P.FACTS):
             try:
                 sig = hb.lower(cfg, ds)
             except UnsupportedPipeline:
                 continue
             c = sig.cfg
-            ref = ref_shim.build_reference(to_plain(cfg), ds)
-            embs = ref.model.embedding_model.embeddings
-            keys = list(to_plain(cfg)["embedding"]["embeddings"].keys())
-            isects = [embs[i].intersect_fn for i, k in enumerate(keys) if cfg.embedding.embeddings[k].type == "ray_intersect"]
-            it = isects[-1]
+            rec = records[(name, fi)]
             S = c.n_samples
-            name = os.path.basename(f)
-            assert torch.equal(torch.tensor(list(c.samples)[:S]), it.samples.reshape(-1).float()), name
-            zs = torch.as_tensor(it.z_scale).reshape(-1).float()
+            assert torch.equal(torch.tensor(list(c.samples)[:S]), torch.tensor(rec["samples"])), name
+            zs = torch.tensor(rec["z_scale"])
             if c.isect_type == L.ISECT_VOXEL:
                 assert torch.equal(torch.tensor(list(c.z_scale3)), zs), name
             else:
                 assert abs(c.z_scale - float(zs[0])) <= 1e-7 * max(1.0, abs(float(zs[0]))), name
             f32 = lambda v: float(torch.tensor(float(v), dtype=torch.float32))  # the struct holds fp32, like the tensors they meet
-            if it.cur_iter <= it.mask_stop_iters:  # otherwise nothing is masked and the bounds are irrelevant
-                assert c.isect_near == f32(it.near) and c.isect_far == f32(it.far), name
+            if rec["masked"]:  # otherwise nothing is masked and the bounds are irrelevant
+                assert c.isect_near == f32(rec["near"]) and c.isect_far == f32(rec["far"]), name
             if c.contract_type == L.CONTRACT_MIPNERF:
-                cf = it.contract_fn
-                assert (c.contract_start_radius, c.contract_end_radius) == (f32(cf.contract_start_radius), f32(cf.contract_end_radius)), name
-                assert (c.contract_start_distance, c.contract_end_distance) == (f32(cf.contract_start_distance), f32(cf.contract_end_distance)), name
+                r0, r1, d0, d1 = rec["contract"]
+                assert (c.contract_start_radius, c.contract_end_radius) == (f32(r0), f32(r1)), name
+                assert (c.contract_start_distance, c.contract_end_distance) == (f32(d0), f32(d1)), name
             if c.cascade:
-                it0 = isects[0]
-                assert torch.equal(torch.tensor(list(c.pre_samples_tab)[:c.pre_samples]), it0.samples.reshape(-1).float()), name
-                assert abs(c.pre_z_scale - float(torch.as_tensor(it0.z_scale).reshape(-1)[0])) <= 1e-7, name
-            net = ref.model.color_model.net
-            assert c.distance_scale == f32(net.distance_scale) and c.weight_thre == f32(net.rayMarch_weight_thres), name
-            assert bool(c.white_bg) == bool(net.white_bg) and bool(c.black_bg) == bool(net.black_bg), name
-            assert [c.aabb[i] for i in range(6)] == [f32(v) for v in net.aabb.reshape(-1)], name
-            assert hb.state.default_grid(sig) == net.gridSize.tolist(), name
+                assert torch.equal(torch.tensor(list(c.pre_samples_tab)[:c.pre_samples]), torch.tensor(rec["pre_samples"])), name
+                assert abs(c.pre_z_scale - rec["pre_z_scale"]) <= 1e-7, name
+            assert c.distance_scale == f32(rec["distance_scale"]) and c.weight_thre == f32(rec["weight_thre"]), name
+            assert bool(c.white_bg) == rec["white_bg"] and bool(c.black_bg) == rec["black_bg"], name
+            assert [c.aabb[i] for i in range(6)] == [f32(v) for v in rec["aabb"]], name
+            assert hb.state.default_grid(sig) == rec["grid"], name
             if c.dynamic:
-                assert (c.num_keyframes, c.num_frames) == (int(net.num_keyframes), int(net.total_num_frames)), name
+                assert [c.num_keyframes, c.num_frames] == rec["frames"], name
             checked += 1
-    assert checked == 90
+    assert checked == len(records) == 90
 
 
 def test_lowered_activations_equal_the_reference_modules_on_every_shipped_yaml():
     """signature.resolve_activation lowers every head / intersect / flow / offset activation to y = f(x * inner + shift) * outer
     (the form the kernels evaluate): the same numbers as the reference's activation modules at render iteration, for every
     activation of all shipped YAMLs that lower."""
-    import glob
-    import os
-
     import hyperreel_b200 as hb
     from hyperreel_b200 import lib as L
     from hyperreel_b200.config import epochs_to_iters, to_plain
     from hyperreel_b200.signature import RENDER_ITER, UnsupportedPipeline, resolve_activation
 
-    ref_shim.install()
-    from nlf.activations import get_activation
-
-    def walk(o, path=""):
-        if isinstance(o, dict):
-            for k, v in o.items():
-                if k.endswith("activation") and (isinstance(v, (dict, str))):
-                    yield path + "/" + k, v
-                if isinstance(v, (dict, list)):
-                    yield from walk(v, path + "/" + k)
-        elif isinstance(o, list):
-            for i, v in enumerate(o):
-                yield from walk(v, f"{path}[{i}]")
-
-    ds = {"num_keyframes": 12, "num_frames": 50, "near": 0.5, "far": 10.0, "depth_range": [0.5, 10.0], "name": "x", "collection": "y",
-          "bbox_min": [-1.5, -1.25, -1.0], "bbox_max": [1.5, 1.25, 1.0], "total_images_per_frame": 5, "val_all": True}
-    x = torch.linspace(-6.0, 6.0, 97)
+    recorded = P.meta("activations")
+    x = P.activation_inputs()
     n = 0
-    for f in sorted(glob.glob(os.path.join(ref_shim.REFERENCE_ROOT, "conf/experiment/model/*.yaml"))):
-        cfg = hb.load_model_yaml(f)
+    for name in sorted(P.model_yamls()):
+        cfg = _yaml(name)
         if cfg is None:
             continue
         try:
-            hb.lower(cfg, ds)
+            hb.lower(cfg, P.DS_R2)
         except UnsupportedPipeline:
             continue
         plain = epochs_to_iters(to_plain(cfg), 1)
-        for path, acfg in walk(plain["embedding"]):
+        for path, acfg in P.walk_activations(plain["embedding"]):
             if isinstance(acfg, dict) and "type" not in acfg:
                 continue
             try:
                 act = resolve_activation(hb.to_cfg(acfg) if isinstance(acfg, dict) else acfg, RENDER_ITER)
             except UnsupportedPipeline:
                 continue  # an activation of an embedding the fused path does not evaluate (e.g. angular flow): never lowered
-            mod = get_activation(ref_shim.to_attr(acfg) if isinstance(acfg, dict) else acfg)
-            if hasattr(mod, "set_iter"):
-                mod.set_iter(RENDER_ITER)
-            want = mod(x.clone())
+            want = torch.tensor(recorded[P.activation_key(acfg)])
             v = x * act.inner_fac + act.shift
             v = torch.sigmoid(v) if act.kind == L.ACT_SIGMOID else (torch.tanh(v) if act.kind == L.ACT_TANH else v)
             got = v * act.outer_fac
-            assert float((got - want).abs().max()) <= 1e-6, (os.path.basename(f), path)
+            assert float((got - want).abs().max()) <= 1e-6, (name, path)
             n += 1
     assert n > 300
